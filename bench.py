@@ -5,12 +5,17 @@ Default workload (BASELINE configs[1], `--config 2`): celeba_hq.yml denoiser (ra
 pooling), sigma_y=0, T_sampling=100, eta=0.85, 16 images per GPU.  A "step" = one full sampling of the per-GPU batch.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5a|5b] [--precision fp32|fp16]
+                    [--dump-outputs DIR]
 
 `value`  : the loop with x_T / y resident in HBM; the per-pair Gaussian draws ARE inside the timed region (drawn chunk by chunk on a
            side stream by ddnm_b200.sampler, like the reference's one randn_like per step).
 `e2e`    : the public drop-in call (ddnm_diffusion / ddnm_plus_diffusion) with pinned HOST x_T / y and CPU results.
 N>1 is launched by torchrun (one rank per GPU): rows shard over ranks, no traffic inside the loop, one all-gather of the restored
 images per step (weak scaling); an untimed sharded-vs-unsharded check runs first (`shard_check`).
+`--dump-outputs DIR`: after the timed steps, the last step's results (restored images `x0`, last x0 prediction `x0_pred`, all
+ranks' rows) go to DIR/<name>.npy as float32, so that two builds can be compared output for output: every input is drawn from fixed
+seeds, so the same arguments give the same inputs.  An output over its share of 64 MB is replaced by a fixed, seeded sample of its
+elements (flattened).
 `--impl reference` times the UNMODIFIED reference (oracle/_ref, see oracle/make_ref.py) on the host cores on a bounded sample.
 The other BASELINE configs (`--config 3|4|5a|5b`) and the fp16 fast mode print the same line for their workload; their results are
 kept under profiles/ (the driver's N=1 line stays configs[1]).
@@ -41,6 +46,21 @@ CONFIGS = {
                workload="celeba_hq.yml simple-UNet + cs_walshhadamard ratio 0.25, sigma_y=0, T_sampling=250, batch 16/GPU (128 over 8 GPUs)"),
 }
 STEP_KERNELS = {"sr4": 1, "color": 1, "inpaint": 1, "wh": 7, "deblur": 13}   # own launches of the fused per-pair update (operators.cu step())
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Write each tensor of `arrays` as dirname/<name>.npy (float32), in all at most DUMP_BYTES: a tensor larger than its share is
+    replaced by the elements at a fixed, seeded set of flat positions (in ascending order), the same in every run."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096          # room for the .npy header
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            idx = np.random.default_rng(1234).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def metric_name(c):
@@ -235,10 +255,14 @@ def main():
     ap.add_argument("--precision", default="fp32", choices=["fp32", "fp16"],
                     help="fp32 = fp32-grade 3x fp16 products (parity mode); fp16 = 1 product per MAC, the analogue of use_fp16 (NOT parity grade)")
     ap.add_argument("--batch", type=int, default=0, help="images per GPU (default: the config's)")
-    ap.add_argument("--e2e-steps", type=int, default=0, help="timed steps of the end-to-end leg (default max(5, steps))")
+    ap.add_argument("--e2e-steps", type=int, default=0, help="timed steps of the end-to-end leg (default: --steps)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-steps", type=int, default=0, help="(ncu runs) skip the e2e / baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args, emit)
     assert args.warmup >= 3 or args.profile_steps, "timing rules: at least 3 warm-up steps"
@@ -329,14 +353,14 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.barrier()
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return ms.item()
+        return ms.item(), out
 
     if args.profile_steps:      # ncu launch list: just run the hot path
         for _ in range(args.profile_steps):
@@ -347,10 +371,19 @@ def main():
 
     clocks = ClockSampler(local)
     clocks.start()
-    ms_total = timed(step_device, args.steps, args.warmup)
+    ms_total, (x0, x0p) = timed(step_device, args.steps, args.warmup)
     clk = clocks.stop()
-    e2e_steps = args.e2e_steps or max(5, args.steps)
-    ms_e2e = timed(step_e2e, e2e_steps, 2)
+    if args.dump_outputs:
+        if world > 1:       # x0 is already every rank's rows; gather the x0 predictions the same way
+            x0 = torch.cat(x0)
+            parts = [torch.empty_like(x0p) for _ in range(world)]
+            dist.all_gather(parts, x0p)
+            x0p = torch.cat(parts)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"x0": x0, "x0_pred": x0p})
+    del x0, x0p
+    e2e_steps = args.e2e_steps or args.steps
+    ms_e2e, _ = timed(step_e2e, e2e_steps, 2)
     ms_step = ms_total / args.steps
     value = Bg * 1e3 / ms_step
     e2e_value = Bg * 1e3 / (ms_e2e / e2e_steps)

@@ -587,7 +587,9 @@ void splitk_reduce(const float* part, int S, long long stride, const View& out, 
                    int ldr, cudaStream_t st) {
   DDNM_CHECK(out.C % 4 == 0 && out.ld % 4 == 0 && S >= 2, "split-K reduce: unsupported shape");
   const int HW = out.H * out.W;
-  const int ppc = std::max(1, (int)cdivll((long long)HW * out.N, 296));
+  // a CTA reduces 2048 values of one image (ppc pixels x C channels): the fp32 grouping of the GroupNorm sums then depends on the
+  // layer's shape only, so a row's result is the same in an engine of any batch size (a ragged last batch rides on a bigger engine)
+  const int ppc = std::max(1, 2048 / out.C);
   dim3 grid(cdiv(HW, ppc), out.N);
   launch_pdl(splitk_reduce_kernel, grid, dim3(std::min(256, out.C / 4)), 0, st, 1, part, S, stride, HW, out.C, out.p, out.ld, chanadd, ca_ld, residual,
              ldr, out.st, out.st_ld, ppc);

@@ -26,6 +26,27 @@ def test_reference_arm_prints_one_json_line():
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0 and "workload" in d["config"]
 
 
+def test_dump_outputs_is_bounded_and_reproducible(tmp_path, monkeypatch):
+    """--dump-outputs: float32 .npy files, at most DUMP_BYTES in all; a small output is written whole, a larger one as the same
+    seeded sample of its elements in every run (so two builds can be compared output for output)."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    small = torch.randn(2, 3, 8, 8, dtype=torch.float64)
+    big = torch.arange(1 << 19, dtype=torch.float32)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"small": small, "big": big})
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["big.npy", "small.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_BYTES
+    s, b = np.load(tmp_path / "a" / "small.npy"), np.load(tmp_path / "a" / "big.npy")
+    assert s.dtype == b.dtype == np.float32 and np.array_equal(s, small.float().numpy())
+    assert 0 < b.size < big.numel() and np.all(np.diff(b) > 0) and np.array_equal(b, big.numpy()[b.astype(np.int64)])
+    assert np.array_equal(b, np.load(tmp_path / "b" / "big.npy"))
+
+
 def test_nonzero_rank_of_reference_arm_exits_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],
